@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Headline benchmark: stencil cell-updates/s and fraction of the HBM roofline (BASELINE.json).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config C] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config C] [--impl ours|reference] [--dump-outputs DIR]
 
 A *step* is one execution of the whole stencil program (all chained operators) over one synthetic
 field.  Default workload = BASELINE.json configs[1]: Jacobi-3D, 8 chained operators, 1024^3 float32,
@@ -15,10 +15,14 @@ fused pass (weak scaling).  The same line also carries
   with the one-GPU time of the same box next to it.
 
 One JSON line is printed by rank 0; see DESIGN.md section "Measurement" for the definition of every key.
+Compiled kernels, generated programs and the CPU oracle's build go to a temporary directory (or to
+``SFB200_CACHE`` if that is set), so the tree this runs from may be read-only.
 """
 import argparse
+import contextlib
 import json
 import os
+import shutil
 import subprocess
 import sys
 import tempfile
@@ -148,6 +152,48 @@ def host_inputs(prog, dims, seed=SEED):
     return out
 
 
+@contextlib.contextmanager
+def scratch_cache():
+    """Points ``SFB200_CACHE`` (NVRTC cubins, generated programs, the oracle's build) at a fresh temporary
+    directory for the duration of the run and removes it afterwards, unless the caller has set it."""
+    if os.environ.get("SFB200_CACHE"):
+        yield
+        return
+    path = tempfile.mkdtemp(prefix="sfb200_bench_")
+    os.environ["SFB200_CACHE"] = path           # inherited by the ranks torchrun starts
+    try:
+        yield
+    finally:
+        shutil.rmtree(path, ignore_errors=True)
+
+
+def oracle_build_dir():
+    cache = os.environ.get("SFB200_CACHE")
+    return os.path.join(cache, "oracle") if cache else None
+
+
+DUMP_BYTES = 32 << 20       # all arrays of --dump-outputs together
+DUMP_SEED = 4321
+
+
+def dump_outputs(program, directory, halo):
+    """``--dump-outputs``: every output field of ``program`` as it is on the device now, written as
+    ``<directory>/<field>.npy`` in the field's data type.  The ``-halo`` border of shrink boundaries is cut
+    off: its content is not defined.  A field larger than its share of DUMP_BYTES is written as its values
+    at distinct flat indices drawn with DUMP_SEED, in ascending order (1-D), the same sample on every run."""
+    os.makedirs(directory, exist_ok=True)
+    outputs = program.program.outputs
+    share = DUMP_BYTES // len(outputs)
+    for name in outputs:
+        arr = program.download(name)
+        if halo:
+            arr = arr[tuple(slice(halo, -halo) for _ in arr.shape)]
+        if arr.nbytes > share:
+            flat = np.unique(np.random.default_rng(DUMP_SEED).integers(0, arr.size, size=share // arr.itemsize))
+            arr = arr[np.unravel_index(flat, arr.shape)]
+        np.save(os.path.join(directory, name + ".npy"), np.ascontiguousarray(arr))
+
+
 # ------------------------------------------------------------------------------------ CPU arm
 
 
@@ -175,7 +221,7 @@ class CpuSample:
         def build(dims):
             p = json.loads(json.dumps(prog))
             p["dimensions"] = dims
-            ref = reference_cpp.CompiledReference(p)
+            ref = reference_cpp.CompiledReference(p, build_dir=oracle_build_dir())
             inputs = {}
             for k, (iname, cfg) in enumerate(p["inputs"].items()):
                 lo, hi = INPUT_RANGES.get(iname, (0.0, 1.0))
@@ -290,7 +336,7 @@ def make_program(index, world, rank, local_rank, comm, scaling):
     from stencilflow_b200 import programs
     from stencilflow_b200.cuda_program import CudaProgram
     name, prog, halo = build_config(index, scale_i=world if scaling == "weak" else 1)
-    path = programs.write_program(prog, name)
+    path = programs.write_program(prog, name, programs.scratch_dir())
     if world > 1:
         from stencilflow_b200 import distributed
         program = distributed.SlabProgram(path, comm, device=local_rank)
@@ -315,15 +361,20 @@ def time_device(program, steps, warmup, comm, sampler=None):
     barrier()
     if sampler is not None:
         sampler.start()
-    launches0 = program.launch_count
-    e0, e1 = rtm.event_create(), rtm.event_create()
-    barrier()
-    rtm.event_record(e0)
-    for _ in range(steps):
-        program.execute()
-    rtm.event_record(e1)
-    rtm.event_synchronize(e1)
-    barrier()
+    try:
+        launches0 = program.launch_count
+        e0, e1 = rtm.event_create(), rtm.event_create()
+        barrier()
+        rtm.event_record(e0)
+        for _ in range(steps):
+            program.execute()
+        rtm.event_record(e1)
+        rtm.event_synchronize(e1)
+        barrier()
+    except BaseException:
+        if sampler is not None:
+            sampler.stop()                  # no nvidia-smi left running behind a failed run
+        raise
     ms_local = rtm.elapsed_ms(e0, e1)
     rtm.event_destroy(e0)
     rtm.event_destroy(e1)
@@ -367,7 +418,7 @@ def verify_single(program, prog, path, index, local_rank, planes=128):
     keep = planes if block < dims[0] else dims[0]
     sub = json.loads(json.dumps(prog))
     sub["dimensions"] = [block] + dims[1:]
-    ref = reference_cpp.CompiledReference(sub)
+    ref = reference_cpp.CompiledReference(sub, build_dir=oracle_build_dir())
     ins = host_inputs(prog, sub["dimensions"])
     expected = ref(**ins)[out_name]
     plane = int(np.prod(f_out.shape[1:]))
@@ -485,7 +536,7 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=100,
-                    help="timed executions of the program (default 100: long enough for the clock "
+                    help="timed executions of the program, at least 1 (default 100: long enough for the clock "
                          "sampler to see the load and for the power cap to show)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--config", type=int, default=1, help="index into BASELINE.json configs")
@@ -502,7 +553,15 @@ def main():
     ap.add_argument("--no-verify", action="store_true")
     ap.add_argument("--no-strong", action="store_true",
                     help="skip the configs[4] strong-scaling block (default: measured when --config 1)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the program's output fields as DIR/<field>.npy "
+                         "(fields above 32 MB as a fixed seeded sample; shrink borders cut off), so that "
+                         "two builds can be compared output for output; --impl ours with one GPU only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.gpus != 1):
+        ap.error("--dump-outputs needs --impl ours and --gpus 1")
     global VARIANT
     VARIANT = args.variant
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
@@ -545,6 +604,8 @@ def main():
     sampler = ClockSampler(local_rank) if rank == 0 else None
     ms_local, ms, launches = time_device(program, args.steps, args.warmup, comm, sampler)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        dump_outputs(program, args.dump_outputs, build_config(args.config)[2])
     per_rank_ms = [t / args.steps for t in time_device.per_rank_ms]
     ms_per_step = ms / args.steps
     value = updates_per_step / (ms_per_step * 1e-3)
@@ -726,4 +787,5 @@ def measure_e2e(program, prog, args, updates_per_step, comm=None):
 
 
 if __name__ == "__main__":
-    main()
+    with scratch_cache():
+        main()

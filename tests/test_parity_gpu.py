@@ -202,6 +202,27 @@ def test_device_utilities(gpu):
     assert not np.array_equal(a, b)
 
 
+def test_bench_dump_outputs_match_oracle(gpu, tmp_path):
+    """``bench.py --dump-outputs`` writes what exactly ``--steps`` timed executions of BASELINE configs[0]
+    computed; it equals the oracle on the same seeded inputs."""
+    import subprocess
+    import sys
+    import bench
+    from oracle import reference_numpy as rn
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--config", "0", "--steps", "2",
+                          "--no-cpu-baseline", "--no-e2e", "--dump-outputs", str(tmp_path / "dump")],
+                         stdout=subprocess.PIPE, text=True, timeout=600, check=True).stdout
+    line = json.loads(out.strip().splitlines()[-1])
+    assert line["steps"] == 2 and line["gpu_launches"] == 2 * line["roofline"]["launches_per_step"]
+    assert line["verify"]["ok"]
+    _, prog, _ = bench.build_config(0)
+    expected = rn.run_reference(prog, bench.host_inputs(prog, prog["dimensions"]))
+    for field, ref in expected.items():
+        got = np.load(tmp_path / "dump" / (field + ".npy"))
+        assert got.dtype == ref.dtype and got.shape == ref.shape
+        assert rn.max_relative_error(ref, got) <= TOL[ref.dtype.name], field
+
+
 def test_size_independent_properties_at_scale(gpu):
     """256^3 x 8 chained Jacobi on hash-generated input, checked by properties that do not need the
     oracle to hold nine 256^3 arrays: linearity and agreement of fused vs unfused execution."""

@@ -251,6 +251,27 @@ def test_reference_arm_line(monkeypatch):
     assert set(line["config"]) == {"workload", "per_gpu", "l2", "input"}
 
 
+def test_bench_dump_outputs_writes_a_fixed_sample(tmp_path):
+    """``bench.py --dump-outputs``: a small output is written whole, a large one as the same seeded sample
+    on every run, all files within the size budget; the undefined -halo border is left out."""
+    import types
+    import numpy as np
+    import bench
+    fields = {"small": np.arange(6 * 7 * 8, dtype=np.float64).reshape(6, 7, 8),
+              "large": np.full((68, 512, 260), np.nan, np.float32)}
+    fields["large"][2:-2, 2:-2, 2:-2] = np.random.default_rng(0).random((64, 508, 256), np.float32)
+    fake = types.SimpleNamespace(program=types.SimpleNamespace(outputs=list(fields)),
+                                 download=lambda name: fields[name].copy())
+    for run in ("a", "b"):
+        bench.dump_outputs(fake, str(tmp_path / run), halo=2)
+    assert np.array_equal(np.load(tmp_path / "a" / "small.npy"), fields["small"][2:-2, 2:-2, 2:-2])
+    large = np.load(tmp_path / "a" / "large.npy")
+    assert large.dtype == np.float32 and large.ndim == 1 and large.size > 1000000
+    assert not np.isnan(large).any()
+    assert np.array_equal(large, np.load(tmp_path / "b" / "large.npy"))
+    assert sum(os.path.getsize(p) for p in (tmp_path / "a").iterdir()) <= 64 << 20
+
+
 def test_choose_chunk_balances_waves_and_warmup():
     from stencilflow_b200.lower_stream import choose_chunk
     # 304 tiles of config 1, 8 warm-up planes per chunk, one CTA per SM
