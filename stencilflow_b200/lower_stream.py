@@ -284,7 +284,31 @@ __device__ __forceinline__ void sf_stp(float* __restrict__ p, const float2* src)
     *reinterpret_cast<SfVec<float, V>*>(p) = t;
 #endif
 }
-"""
+// ---- tensor memory (tcgen05, cta_group::1): one warp allocates all 512 columns for the CTA; each thread then
+// moves 32-bit words between its registers and its own lane of the columns (shape 32x32b)
+__device__ __forceinline__ void sf_tmem_alloc(u32* dst) {
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 512;" ::"r"(sf_smem_addr(dst)) : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+}
+__device__ __forceinline__ void sf_tmem_dealloc(u32 base) {
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" ::"r"(base) : "memory");
+}
+__device__ __forceinline__ void sf_tmem_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
+__device__ __forceinline__ void sf_tmem_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
+__device__ __forceinline__ void sf_tmem_wait_st() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
+__device__ __forceinline__ void sf_tmem_wait_ld() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
+""" + "".join(
+    '__device__ __forceinline__ void sf_tmem_st{n}(u32 a, {decl}) {{\n'
+    '    asm volatile("tcgen05.st.sync.aligned.32x32b.x{n}.b32 [%0], {{{regs}}};" ::"r"(a), {ops} : "memory");\n}}\n'
+    '__device__ __forceinline__ void sf_tmem_ld{n}(u32 a, {rdecl}) {{\n'
+    '    asm volatile("tcgen05.ld.sync.aligned.32x32b.x{n}.b32 {{{lregs}}}, [%{n}];" : {lops} : "r"(a) : "memory");\n}}\n'.format(
+        n=n, decl=", ".join("u32 v{}".format(i) for i in range(n)),
+        regs=",".join("%{}".format(i + 1) for i in range(n)),
+        ops=", ".join('"r"(v{})'.format(i) for i in range(n)),
+        rdecl=", ".join("u32& v{}".format(i) for i in range(n)),
+        lregs=",".join("%{}".format(i) for i in range(n)),
+        lops=", ".join('"=r"(v{})'.format(i) for i in range(n)))
+    for n in (1, 2, 4, 8, 16))
 
 
 def l2_hint_defines():
@@ -449,6 +473,7 @@ class GroupAnalysis:
         if not any(i.kind == "ext" for i in self.fields.values()):
             raise NotStreamable("group reads no full-dimensional field")
         self._lags()
+        self.tmem_ages = self._tmem_slots()
         self._halos()
         spos = 3 - self.ndim                      # position of the streamed iterator in (i, j, k)
         for op in ops:
@@ -514,6 +539,23 @@ class GroupAnalysis:
                 f[field].back = max(f[field].back, f[op.name].back + max(0, -d))
                 f[field].fwd = max(f[field].fwd, f[op.name].fwd + max(0, d))
 
+    def _tmem_slots(self):
+        """{field: age} of the window slots that may wait in tensor memory between two uses.  The oldest plane of
+        a window (age window - 1) qualifies when every read of it at that age is an own-cell tap (dj == dk == 0):
+        no shuffle and no exchange ring reads it, only the thread that holds it.  Its owner parks it after its
+        last use one step younger and fetches it back a step later, so its registers are free in between."""
+        f = self.fields
+        out = collections.OrderedDict()
+        for name, info in f.items():
+            age = info.window - 1
+            if not info.consumed or age < 1:
+                continue
+            reads = [(dj, dk) for op in self.ops for (field, d, dj, dk) in self.taps[op.name]
+                     if field == name and f[op.name].lag - d - info.lag == age]
+            if reads and all(dj == 0 and dk == 0 for (dj, dk) in reads):
+                out[name] = age
+        return out
+
     def _halos(self):
         f = self.fields
         for op in reversed(self.ops):
@@ -547,14 +589,17 @@ class GroupAnalysis:
         per = self.dtype.bytes // 4
         return sum(i.window for i in self.fields.values() if i.consumed) * R * V * per
 
-    def register_estimate(self, R, V):
+    def register_estimate(self, R, V, tmem=False):
         """Registers per thread the generated kernel needs: the planes of every window that are
         live across steps (the oldest plane of a window dies while the newest is being produced)
         plus what is in flight -- the plane being produced, its consumer's result, the pre-fetched
         neighbour cells of the next operator, addresses, masks and loop state.  The constant part is
-        fitted to ptxas' allocations of the Jacobi/hdiff kernels (spill-free iff estimate <= limit)."""
+        fitted to ptxas' allocations of the Jacobi/hdiff kernels (spill-free iff estimate <= limit).
+        ``tmem``: the slots of ``tmem_ages`` wait in tensor memory, not in registers, across a step."""
         per = self.dtype.bytes // 4
         live = sum(max(1, i.window - 1) for i in self.fields.values() if i.consumed)
+        if tmem:
+            live -= len(self.tmem_ages)
         hoisted = 0
         for (field, off) in self.aux_hoisted():
             _, dr, dc = self.aux_split(off)
@@ -572,7 +617,7 @@ class GroupAnalysis:
 
 
 class Geometry:
-    def __init__(self, ana: GroupAnalysis, V, R, WR, WC, prefetch, KS=32, sync="cta", direct=False):
+    def __init__(self, ana: GroupAnalysis, V, R, WR, WC, prefetch, KS=32, sync="cta", direct=False, tmem=False):
         """``KS`` = threads per tile row.  32 (a warp per row, k-neighbours by shuffle) in general;
         for groups without k-taps on a narrow innermost dimension the whole extent is one row of
         ``KS = NK / V`` threads and thread t owns row group t / KS ("flat lanes": no idle lanes)."""
@@ -644,6 +689,21 @@ class Geometry:
         if self.halves:
             self.box = [self.box_cols, self.TR // 2, 1]
         self.smem = self._smem(ana)
+        # tensor memory: the window slots of ``ana.tmem_ages`` wait there between two uses (StreamKernelGen).  The
+        # CTA allocates all 512 columns, so it must be alone on its SM; warp w reaches TMEM lanes 32 (w % 4) ...
+        # + 31 and owns 128 columns of them (at most 16 warps), two planes per slot, each padded to a power of two
+        self.tmem_cols = 0
+        if tmem and ana.ndim == 3 and ana.tmem_ages and nw <= 16:
+            words = R * V * ana.dtype.bytes // 4
+            self.tmem_cols = 1 << (words - 1).bit_length()
+            if 2 * self.tmem_cols * len(ana.tmem_ages) > 128:
+                self.tmem_cols = 0
+        self.tmem = bool(self.tmem_cols)
+        if self.tmem:
+            self.tmem_off = self.smem          # the address tcgen05.alloc returns
+            self.smem += 16
+            if resident_estimate(self) != 1:
+                self.tmem, self.tmem_cols, self.smem = False, 0, self.tmem_off
 
     def _smem(self, ana):
         b = ana.dtype.bytes
@@ -745,6 +805,10 @@ class StreamKernelGen:
         if self.flags:
             self.split_barrier = False
         self._waited = set()
+        # tensor memory (Geometry.tmem): the two planes of a slot in flight alternate between two column sets, so
+        # the unrolled loop needs an even number of steps and static window slots
+        self.tmem = bool(geo.tmem and self.U % 2 == 0 and all(self.wperiod(ana.fields[n]) for n in ana.tmem_ages))
+        self._tm_loaded, self._tm_waited = set(), set()
         self.rotate_rows, self.skip_warps, self.skip_from = self._halo_warps()
         self.ops_limit = len(ops)
         # how produced planes get their out-of-domain cells set to the boundary value (see _finish_field)
@@ -977,6 +1041,10 @@ class StreamKernelGen:
             e("unsigned long long* const sbar = reinterpret_cast<unsigned long long*>(sf_smem + {});".format(g.sbar_off))
             if U % 2:
                 e("u32 sphase = 0;")
+        if self.tmem:
+            e("u32* const sf_tmem = reinterpret_cast<u32*>(sf_smem + {});".format(g.tmem_off))
+            if self.persistent:
+                self._emit_tmem_alloc()
 
         # ---- the segment(s) this CTA streams: a tile and a range of planes of the streamed dimension
         gx = -(-self.NK // g.BK)
@@ -1007,6 +1075,8 @@ class StreamKernelGen:
             e("const int c_begin = s_begin + blockIdx.z * chunk;")
             e("const int c_end = min(c_begin + chunk, s_end);")
             e("if (c_begin >= c_end) return;")
+            if self.tmem:
+                self._emit_tmem_alloc()
         e("const int gk = tile_k0 - {} + c0;                 // global k of the first owned column".format(g.HK0))
         if ndim == 3:
             e("const int gj0 = tile_j0 - {} + r0;".format(g.HJ0))
@@ -1217,6 +1287,11 @@ class StreamKernelGen:
             e("__threadfence();", 2)
             e("if (atomicAdd(&work_tab[1], 1) == (int)gridDim.x - 1) { work_tab[0] = 0; work_tab[1] = 0; __threadfence(); }", 2)
             e("}")
+        if self.tmem:
+            e("sf_tmem_wait_st();")
+            e("sf_tmem_fence_before();")
+            e("__syncthreads();")
+            e("if (warp_u == 0) { sf_tmem_fence_after(); sf_tmem_dealloc(*sf_tmem); }")
         body = "\n".join(self.lines)
         digest = hashlib.sha1((body + ";".join(params)).encode()).hexdigest()[:12]
         name = "sf_stream_{}".format(digest)
@@ -1230,6 +1305,89 @@ class StreamKernelGen:
         if self.peer_push:
             args += [("push", i.name) for i in stored]
         return name, src, args
+
+    def _emit_tmem_alloc(self):
+        """Warp 0 allocates the 512 columns; every warp then owns 128 of them in its lane quarter."""
+        e = self.emit
+        e("if (warp_u == 0) sf_tmem_alloc(sf_tmem);")
+        e("sf_tmem_fence_before();")
+        e("__syncthreads();")
+        e("sf_tmem_fence_after();")
+        e("const u32 tm_base = *sf_tmem + ((u32)(32 * (warp_u % 4)) << 16) + (u32)(warp_u / 4) * 128;")
+
+    def _tm_words(self, info, slot):
+        """(C lvalues of the cells of a window slot, 32-bit words of them in column order)"""
+        g = self.geo
+        cells = [self.cellref("w_{}[{}][{}]".format(self.fid[info.name], slot, r), v)
+                 for r in range(g.R) for v in range(g.V)]
+        if self.ct == dtypes.float32:
+            return cells, ["__float_as_uint({})".format(c) for c in cells]
+        return cells, [w for c in cells for w in ("(u32)__double2loint({})".format(c), "(u32)__double2hiint({})".format(c))]
+
+    def _tm_chunks(self, n):
+        pos = 0
+        for size in (16, 8, 4, 2, 1):
+            while n - pos >= size:
+                yield pos, size
+                pos += size
+
+    def _tm_column(self, name, parity):
+        return "tm_base + {}".format((2 * list(self.ana.tmem_ages).index(name) + parity) * self.geo.tmem_cols)
+
+    def _tm_store(self, info, u):
+        """Parks the plane that is one step younger than the field's TMEM slot (its last use is behind it)."""
+        age = self.ana.tmem_ages[info.name]
+        cells, words = self._tm_words(info, self.wslot(info, age - 1, u))
+        col = self._tm_column(info.name, (u - age + 1) % 2)
+        for pos, n in self._tm_chunks(len(words)):
+            self.emit("sf_tmem_st{}({} + {}, {});".format(n, col, pos, ", ".join(words[pos:pos + n])), 2)
+
+    def _tm_load(self, info, u):
+        """Fetches the field's TMEM slot back into its window registers (valid after _tm_wait)."""
+        e = self.emit
+        age = self.ana.tmem_ages[info.name]
+        cells, words = self._tm_words(info, self.wslot(info, age, u))
+        col = self._tm_column(info.name, (u - age) % 2)
+        e("{", 3)
+        e("u32 tl[{}];".format(len(words)), 4)
+        for pos, n in self._tm_chunks(len(words)):
+            e("sf_tmem_ld{}({} + {}, {});".format(n, col, pos, ", ".join("tl[{}]".format(pos + i) for i in range(n))), 4)
+        for i, c in enumerate(cells):
+            if self.ct == dtypes.float32:
+                e("{} = __uint_as_float(tl[{}]);".format(c, i), 4)
+            else:
+                e("{} = __hiloint2double((int)tl[{}], (int)tl[{}]);".format(c, 2 * i + 1, 2 * i), 4)
+        e("}", 3)
+
+    def _tm_wait(self, info, u):
+        """tcgen05.wait::ld, then an empty asm that takes the loaded registers through it, so that the
+        compiler does not move their first use above the wait"""
+        age = self.ana.tmem_ages[info.name]
+        cells, _ = self._tm_words(info, self.wslot(info, age, u))
+        self.emit("sf_tmem_wait_ld();", 3)
+        c = "f" if self.ct == dtypes.float32 else "d"
+        for pos in range(0, len(cells), 16):
+            self.emit("asm volatile(\"\" : {});".format(", ".join('"+{}"({})'.format(c, x) for x in cells[pos:pos + 16])), 3)
+
+    def _tm_store_points(self, ops):
+        """{position: [fields]} where the step parks each TMEM field: after the last of ``ops`` that reads the
+        plane one step younger than its slot (k), after the streamed inputs (-1) or at the start of the step (-2)"""
+        a = self.ana
+        out = collections.defaultdict(list)
+        names = [op.name for op in ops]
+        for name, age in (a.tmem_ages.items() if self.tmem else []):
+            src = a.fields[name]
+            readers = [k for k, op in enumerate(ops) for (f, d, dj, dk) in a.taps[op.name]
+                       if f == name and a.fields[op.name].lag - d - src.lag == age - 1]
+            if readers:
+                out[max(readers)].append(src)
+            elif age > 1:
+                out[-2].append(src)
+            elif src.kind == "ext":
+                out[-1].append(src)
+            elif name in names:
+                out[names.index(name)].append(src)
+        return out
 
     def _needs_fixup(self, info):
         """Cells outside the domain must read as the boundary value.  Input planes arrive through TMA,
@@ -1252,6 +1410,10 @@ class StreamKernelGen:
                 nxt = "(slot + {P}) % {D}".format(P=g.P, D=g.D)
                 ph = "phase"
             self._waited = set()
+            self._tm_loaded, self._tm_waited = set(), set()
+            if self.tmem:
+                # the stores of the previous step land before this step fetches what they parked
+                e("sf_tmem_wait_st();", 2)
             if self.flags:
                 # every warp has read its rows of the plane in the TMA slot about to be refilled once it has
                 # published them: the arrivals of the previous step on the streamed inputs' barriers
@@ -1292,12 +1454,17 @@ class StreamKernelGen:
         g, a, e = self.geo, self.ana, self.emit
         ops = self.ops[:n_ops]
         gathered = {}
+        tm_store = self._tm_store_points(ops)
+        for info in tm_store.get(-2, []):
+            self._tm_store(info, u)
         if ops and self.pipeline and self._can_gather_early(ops[0]):
             # neighbour data of the first operator is a step old: fetch it while the TMA lands
             gathered[0] = self._gather_op(ops[0], u, 0)
         e("sf_mbar_wait(&wbars[{}], {});".format(self.slot_expr, ph), 2)
         for i in ext:
             self._produce_ext(i, u)
+        for info in tm_store.get(-1, []):
+            self._tm_store(info, u)
         last_comm = len(self.lines)
         for k, op in enumerate(ops):
             if k not in gathered:
@@ -1309,6 +1476,8 @@ class StreamKernelGen:
                 gathered[k + 1] = self._gather_op(ops[k + 1], u, k + 1)
                 last_comm = len(self.lines)
             self._produce_op(op, u, gathered.pop(k))
+            for src in tm_store.get(k, []):
+                self._tm_store(src, u)
             info = a.fields[op.name]
             if info.consumed and (info.row_ring or info.col_ring):
                 last_comm = len(self.lines)
@@ -1559,6 +1728,9 @@ class StreamKernelGen:
             src = a.fields[field]
             f = self.fid[field]
             tag = "o{}_{}_{}_{}".format(k, f, age, _fmt_off(rr))
+            if self.tmem and a.tmem_ages.get(field) == age and field not in self._tm_loaded:
+                self._tm_loaded.add(field)
+                self._tm_load(src, u)
             if not (0 <= rr < R) or (src.col_ring and (nl or nr)):
                 self._flag_wait(src, age, u, 3)
             if 0 <= rr < R:
@@ -1676,6 +1848,10 @@ class StreamKernelGen:
             else:
                 self.aux_cur[(field, off)] = self._emit_aux_load(field, off, "(" + plane + ")", "ay{}".format(n), 3)
         self._open_plane(info, u)
+        for (field, age, rr) in rows:
+            if self.tmem and a.tmem_ages.get(field) == age and field not in self._tm_waited:
+                self._tm_waited.add(field)
+                self._tm_wait(a.fields[field], u)
         if self.G == 1:
             self._emit_scalar_cells(op, tap_key, tap_cell)
         else:
@@ -2105,13 +2281,23 @@ def choose_geometry(program, ops, options):
                 for prefetch in prefetches:
                     try:
                         ana = GroupAnalysis(program, ops, exchange_cols=(WC > 1))
-                        geo = Geometry(ana, V, R, WR, WC, prefetch, KS, getattr(opts, "sync", "") or DEFAULT_SYNC,
-                                       direct=bool(getattr(opts, "direct", 0)))
+                        sync = getattr(opts, "sync", "") or DEFAULT_SYNC
+                        direct = bool(getattr(opts, "direct", 0))
+                        geo = Geometry(ana, V, R, WR, WC, prefetch, KS, sync, direct=direct,
+                                       tmem=bool(getattr(opts, "tmem", 0)))
+                        if geo.tmem and ana.register_estimate(R, V) < register_limit(geo.NT):
+                            # the windows fit the registers: nothing to park
+                            geo = Geometry(ana, V, R, WR, WC, prefetch, KS, sync, direct=direct)
+                        elif geo.tmem and not getattr(opts, "sync", ""):
+                            # a pass at its register limit spends what the parked planes free on per-field
+                            # mbarriers instead of the CTA barrier (Jacobi-3D 1024^3: 3.69 vs 3.84 ms; parked
+                            # planes under the CTA barrier alone: 4.04 ms, profiles/r03_sweep_tmem_config1.txt)
+                            geo = Geometry(ana, V, R, WR, WC, prefetch, KS, "flags", direct=direct, tmem=True)
                     except NotStreamable:
                         break
                     if geo.smem > SMEM_LIMIT:
                         continue
-                    if not explicit and ana.register_estimate(R, V) > register_limit(geo.NT) + REG_SLACK:
+                    if not explicit and ana.register_estimate(R, V, geo.tmem) > register_limit(geo.NT) + REG_SLACK:
                         continue
                     t = modelled_time(program, ops, ana, geo)
                     if len(program.shape) == 3 and len(prefetches) > 1:
@@ -2420,7 +2606,8 @@ def lower_group(lowered: LoweredProgram, ops: List[StencilOp], options, speciali
                               "tiles": gx * gy, "sync": "pair" if geo.pair else ("halves" if geo.halves else ("flags" if gen.flags else "cta")), "direct": sorted(geo.direct), "unroll": gen.U, "packed": gen.G == 2, "halo_skip": [gen.rotate_rows, gen.skip_warps, gen.skip_from], "lags": {n: i.lag for n, i in ana.fields.items()},
                               "windows": {n: i.window for n, i in ana.fields.items() if i.consumed},
                               "window_registers": ana.window_registers(geo.R, geo.V),
-                              "register_estimate": ana.register_estimate(geo.R, geo.V),
+                              "register_estimate": ana.register_estimate(geo.R, geo.V, geo.tmem),
+                              "tmem": dict(ana.tmem_ages) if gen.tmem else {},
                               "stream_overhead_planes": overhead,
                               "back": max(i.back for i in ana.fields.values()),
                               "reach": reach,

@@ -30,6 +30,8 @@ from . import lower_cuda
 from .stencil_op import StencilProgram
 
 
+# default of PlanOptions.tmem (SFB200_TMEM): park window planes in tensor memory where a 3-D pass needs the registers
+TMEM_DEFAULT = "1"
 TUNED_PLANS = os.path.join(os.path.dirname(os.path.abspath(__file__)), "tuned_plans.json")
 
 
@@ -95,13 +97,15 @@ class PlanOptions:
     measured plans (``tuned_plans.json``) before falling back on the cost model."""
 
     KNOBS = ("SFB200_FUSE", "SFB200_MAX_DEPTH", "SFB200_ROWS", "SFB200_WARPS", "SFB200_CHUNK", "SFB200_PREFETCH",
-             "SFB200_VEC", "SFB200_KS", "SFB200_SYNC", "SFB200_DIRECT")
+             "SFB200_VEC", "SFB200_KS", "SFB200_SYNC", "SFB200_DIRECT",
+             "SFB200_TMEM")
 
     def __init__(self, fuse=None, max_depth=None, rows_per_thread=None, warps=None, chunk=None,
-                 prefetch=None, vector=None, threads_per_row=None, sync=None, direct=None, peer_push=None):
+                 prefetch=None, vector=None, threads_per_row=None, sync=None, direct=None, tmem=None,
+                 peer_push=None):
         env = os.environ
         self.is_default = (all(v is None for v in (fuse, max_depth, rows_per_thread, warps, chunk, prefetch, vector,
-                                                   threads_per_row, sync, direct))
+                                                   threads_per_row, sync, direct, tmem))
                            and not any(k in env for k in self.KNOBS) and env.get("SFB200_TUNED", "1") != "0")
         self.vector = int(env.get("SFB200_VEC", "0")) if vector is None else vector
         self.threads_per_row = int(env.get("SFB200_KS", "0")) if threads_per_row is None else threads_per_row
@@ -115,6 +119,9 @@ class PlanOptions:
         # 1: neighbour rows of a streamed *input* field are read straight from its TMA ring (which then
         # keeps a plane one step longer) instead of being re-published through an exchange ring
         self.direct = int(env.get("SFB200_DIRECT", "0")) if direct is None else int(direct)
+        # 1: 3-D passes with one CTA per SM that sit at their register limit park the oldest plane of a window in
+        # tensor memory between its last use as a centre plane and its use as an own-cell operand
+        self.tmem = int(env.get("SFB200_TMEM", TMEM_DEFAULT)) if tmem is None else int(tmem)
         # slab mode (set by distributed.SlabProgram): streamed kernels store the edge planes of their
         # results straight into the neighbouring GPUs' halo planes.  Not a tuning knob: it does not
         # take part in ``is_default`` and survives the replacement of the options by a measured plan.
