@@ -2283,10 +2283,11 @@ def choose_geometry(program, ops, options):
                         ana = GroupAnalysis(program, ops, exchange_cols=(WC > 1))
                         sync = getattr(opts, "sync", "") or DEFAULT_SYNC
                         direct = bool(getattr(opts, "direct", 0))
-                        geo = Geometry(ana, V, R, WR, WC, prefetch, KS, sync, direct=direct,
-                                       tmem=bool(getattr(opts, "tmem", 0)))
-                        if geo.tmem and ana.register_estimate(R, V) < register_limit(geo.NT):
-                            # the windows fit the registers: nothing to park
+                        tmem = int(getattr(opts, "tmem", 0) or 0)
+                        geo = Geometry(ana, V, R, WR, WC, prefetch, KS, sync, direct=direct, tmem=bool(tmem))
+                        if geo.tmem and tmem < 2 and ana.register_estimate(R, V) < register_limit(geo.NT):
+                            # the windows fit the registers: nothing to park (tmem = 2 parks all the same, so
+                            # that the tensor-memory code of passes far from their register limit can be tested)
                             geo = Geometry(ana, V, R, WR, WC, prefetch, KS, sync, direct=direct)
                         elif geo.tmem and not getattr(opts, "sync", ""):
                             # a pass at its register limit spends what the parked planes free on per-field
@@ -2608,6 +2609,8 @@ def lower_group(lowered: LoweredProgram, ops: List[StencilOp], options, speciali
                               "window_registers": ana.window_registers(geo.R, geo.V),
                               "register_estimate": ana.register_estimate(geo.R, geo.V, geo.tmem),
                               "tmem": dict(ana.tmem_ages) if gen.tmem else {},
+                              # where a step parks each of them: after operator k, -1 after the inputs, -2 first
+                              "tmem_store": {f.name: k for k, fs in gen._tm_store_points(ops).items() for f in fs},
                               "stream_overhead_planes": overhead,
                               "back": max(i.back for i in ana.fields.values()),
                               "reach": reach,

@@ -120,7 +120,8 @@ class PlanOptions:
         # keeps a plane one step longer) instead of being re-published through an exchange ring
         self.direct = int(env.get("SFB200_DIRECT", "0")) if direct is None else int(direct)
         # 1: 3-D passes with one CTA per SM that sit at their register limit park the oldest plane of a window in
-        # tensor memory between its last use as a centre plane and its use as an own-cell operand
+        # tensor memory between its last use as a centre plane and its use as an own-cell operand; 2: park every
+        # slot that qualifies, whatever the register estimate (tests); 0: never
         self.tmem = int(env.get("SFB200_TMEM", TMEM_DEFAULT)) if tmem is None else int(tmem)
         # slab mode (set by distributed.SlabProgram): streamed kernels store the edge planes of their
         # results straight into the neighbouring GPUs' halo planes.  Not a tuning knob: it does not

@@ -6,9 +6,13 @@ from conftest import program_path
 
 
 def _program(name):
+    return _program_at(program_path(name))
+
+
+def _program_at(path):
     from stencilflow_b200.kernel_chain_graph import KernelChainGraph
     from stencilflow_b200.stencil_op import make_program
-    return make_program(KernelChainGraph(program_path(name)))
+    return make_program(KernelChainGraph(path))
 
 
 def _analysis(prog, ops=None):
@@ -100,3 +104,108 @@ def test_generated_pass_allocates_parks_fetches_and_frees():
     off = lower_stream.StreamKernelGen(prog, ops, ana, lower_stream.Geometry(ana, 4, 3, 24, 1, 5, 16),
                                        persistent=True).generate()[1]
     assert "sf_tmem" not in off
+
+
+def _streamed(prog, **opts):
+    from stencilflow_b200 import planner
+    plan = planner.plan_program(prog, planner.PlanOptions(**opts) if opts else None)
+    return [l for l in plan.lowered.launches if l.family == "streamed"]
+
+
+def test_tmem_knob_reaches_the_generator():
+    """diamond3d sits far below the register limit: tmem=1 keeps its planes in registers, tmem=2 parks them all the
+    same, tmem=0 never parks; on the Jacobi-3D pass of config 1 (at its register limit) only tmem=0 keeps them."""
+    geo = dict(max_depth=4, rows_per_thread=4, warps=8, threads_per_row=32, prefetch=2, sync="cta")
+    prog = _program("diamond3d_12x10x16")
+    assert [l.info["tmem"] for l in _streamed(prog, tmem=2, **geo)] == [{"a": 2, "r": 2}]
+    assert [l.info["tmem_store"] for l in _streamed(prog, tmem=2, **geo)] == [{"a": 2, "r": -2}]
+    assert [l.info["tmem"] for l in _streamed(prog, tmem=1, **geo)] == [{}]
+    assert [l.info["tmem"] for l in _streamed(prog, tmem=0, **geo)] == [{}]
+    # the register estimate, not the knob, decides at 1: 12 warps x 3 rows of config 1 parks, with the mbarriers
+    config1 = dict(max_depth=4, rows_per_thread=3, warps=12, prefetch=5)
+    prog = _program("ref_jacobi3d_32x32x32_8itr_8vec")
+    on = _streamed(prog, tmem=1, **config1)
+    assert [l.info["tmem"] for l in on] == [{"a": 2, "b0": 2, "b1": 2, "b2": 2}, {"b3": 2, "b4": 2, "b5": 2, "b6": 2}]
+    assert all(l.info["sync"] == "flags" for l in on)
+    assert not any(l.info["tmem"] for l in _streamed(prog, tmem=0, **config1))
+
+
+def test_tmem_knob_from_the_environment(monkeypatch):
+    from stencilflow_b200.planner import PlanOptions
+    for value in ("0", "1", "2"):
+        monkeypatch.setenv("SFB200_TMEM", value)
+        assert PlanOptions().tmem == int(value) and not PlanOptions().is_default
+    monkeypatch.delenv("SFB200_TMEM")
+    assert PlanOptions().tmem == 1
+
+
+@pytest.mark.parametrize("index,parked", [(1, True), (2, False), (3, False), (4, True)])
+def test_default_plans_of_the_baseline_configs(monkeypatch, index, parked):
+    """The cost model's policy: the Jacobi-3D passes of configs 1 and 4 park their planes and synchronise by
+    per-field mbarriers; hdiff (config 2) and the 2-D chain (config 3) keep every plane in registers."""
+    from stencilflow_b200 import programs
+    from stencilflow_b200.planner import PlanOptions
+    for knob in PlanOptions.KNOBS + ("SFB200_TUNED", "SFB200_PERSISTENT"):
+        monkeypatch.delenv(knob, raising=False)
+    name, prog, _ = programs.baseline_config(index)
+    streamed = _streamed(_program_at(programs.write_program(prog, name)))
+    assert streamed
+    if parked:
+        assert all(l.info["tmem"] and l.info["sync"] == "flags" for l in streamed)
+    else:
+        assert not any(l.info["tmem"] for l in streamed)
+
+
+def test_gpu_matrix_covers_every_parking_shape(monkeypatch):
+    """The GPU matrix of ``test_tmem_gpu.py``, lowered here: every entry parks what it says it parks, and together the
+    entries reach every branch of the generator's parking code -- a slot parked at the start of the step (-2) and
+    after an operator (>= 0), an age-3 slot, two fields parked at one point, float32 and float64, the chunk grid and
+    persistent CTAs, and each synchronisation scheme.  Pruning the matrix must not drop one of them unnoticed."""
+    import test_tmem_gpu as gm
+    seen = set()
+    for name, opts, env, slots in gm.MATRIX:
+        for knob in ("SFB200_PERSISTENT", "SFB200_HALO_SKIP", "SFB200_SPLITLOOP"):
+            monkeypatch.delenv(knob, raising=False)
+        for k, v in env.items():
+            monkeypatch.setenv(k, v)
+        prog = _program_at(gm.case_path(name))
+        assert [l.info["tmem"] for l in _streamed(prog, tmem=0, **opts)] == [{}] * len(slots), (name, opts, env)
+        on = _streamed(prog, tmem=2, **opts)
+        assert [l.info["tmem"] for l in on] == slots, (name, opts, env)
+        dtype = prog.ops[0].data_type.name
+        for l in on:
+            info = l.info
+            if not info["tmem"]:
+                continue
+            points = list(info["tmem_store"].values())
+            seen.update(("store", "start" if k == -2 else ("input" if k == -1 else "op")) for k in points)
+            seen.update(("age", a) for a in info["tmem"].values())
+            if len(points) > len(set(points)):
+                seen.add("shared store point")
+            seen.add(dtype)
+            seen.add("persistent" if info["persistent"] else "chunk grid")
+            seen.add(info["sync"])
+            if info["direct"]:
+                seen.add("direct")
+            if info["halo_skip"][2] < len(l.ops):
+                seen.add("halo warps")
+    need = {("store", "start"), ("store", "op"), ("age", 1), ("age", 2), ("age", 3), "shared store point",
+            "float32", "float64", "persistent", "chunk grid", "cta", "pair", "flags", "halves", "direct", "halo warps"}
+    assert need <= seen, sorted(map(str, need - seen))
+
+
+def test_chunk_grid_allocates_after_its_early_return(monkeypatch):
+    """A CTA of the one-per-(tile, chunk) grid whose chunk is empty leaves before it allocates tensor memory; every
+    other one frees its columns once, at the end."""
+    from stencilflow_b200 import lower_stream
+    monkeypatch.setenv("SFB200_PERSISTENT", "0")
+    prog = _config1()
+    ops = list(prog.ops)[:4]
+    ana = _analysis(prog, ops)
+    geo = lower_stream.Geometry(ana, 4, 3, 24, 1, 5, 16, "flags", tmem=True)
+    gen = lower_stream.StreamKernelGen(prog, ops, ana, geo)
+    _, src, _ = gen.generate()
+    assert gen.tmem and not gen.persistent
+    assert src.count("sf_tmem_alloc(") == 1 and src.count("sf_tmem_dealloc(") == 1
+    assert src.index("if (c_begin >= c_end) return;") < src.index("sf_tmem_alloc(") < src.index("sf_tmem_dealloc(")
+    assert "return;" not in src[src.index("sf_tmem_alloc("):]
