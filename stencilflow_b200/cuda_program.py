@@ -475,12 +475,12 @@ class CudaProgram:
 
         Returns a list of steps ``{"h2d": [(field, b, e)], "launch": [(launch index, b, e)], "d2h":
         [(field, b, e)]}`` (plane ranges along the slab axis, global numbering), or None when the plan
-        cannot be cut: no slab axis, an array that does not span it,
+        cannot be cut: no slab axis, a cluster plan (one launch computes the whole program), an array that does not span it,
         intermediates that share storage (a later piece would still need planes an earlier piece's
         successor overwrote), or a slab whose halo is thinner than the accumulated reach."""
         lowered = self.lowered
         axis = lowered.slab_axis
-        if axis is None or pieces < 2:
+        if axis is None or pieces < 2 or any(l.family == "cluster" for l in lowered.launches):
             return None
         it = "ijk"[axis]
         fields = self.program.fields

@@ -398,6 +398,7 @@ class SlabProgram:
         # rest of the pass, but its kernel variant runs 6-15 % slower than the plain one (same loop, a less
         # lucky register assignment: 4.21-4.57 vs 3.96 ms per step at N = 4, profiles/r02d_push_kinds.txt)
         plan_options.peer_push = comm.world > 1 and os.environ.get("SFB200_PEER_PUSH", PEER_PUSH_DEFAULT) != "0"
+        plan_options.cluster = 0            # a thread-block cluster is one GPU's
         probe = planner.plan_program(make_program(chain), options=plan_options)
         axis = probe.lowered.slab_axis
         if axis is None:

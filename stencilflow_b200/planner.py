@@ -102,7 +102,7 @@ class PlanOptions:
 
     def __init__(self, fuse=None, max_depth=None, rows_per_thread=None, warps=None, chunk=None,
                  prefetch=None, vector=None, threads_per_row=None, sync=None, direct=None, tmem=None,
-                 peer_push=None):
+                 peer_push=None, cluster=None):
         env = os.environ
         self.is_default = (all(v is None for v in (fuse, max_depth, rows_per_thread, warps, chunk, prefetch, vector,
                                                    threads_per_row, sync, direct, tmem))
@@ -123,6 +123,11 @@ class PlanOptions:
         # tensor memory between its last use as a centre plane and its use as an own-cell operand; 2: park every
         # slot that qualifies, whatever the register estimate (tests); 0: never
         self.tmem = int(env.get("SFB200_TMEM", TMEM_DEFAULT)) if tmem is None else int(tmem)
+        # 1: a program whose fields fit the distributed shared memory of one 8-CTA cluster runs as one launch of
+        # the cluster family (lower_cluster); 0: never.  Like ``peer_push`` not a tuning knob: it does not take
+        # part in ``is_default`` and survives the replacement of the options by a measured plan.  Ignored with
+        # fuse=False and in slab mode.
+        self.cluster = int(env.get("SFB200_CLUSTER", "0")) if cluster is None else int(cluster)
         # slab mode (set by distributed.SlabProgram): streamed kernels store the edge planes of their
         # results straight into the neighbouring GPUs' halo planes.  Not a tuning knob: it does not
         # take part in ``is_default`` and survives the replacement of the options by a measured plan.
@@ -130,6 +135,47 @@ class PlanOptions:
 
     def as_dict(self):
         return {k: v for k, v in self.__dict__.items() if k != "is_default"}
+
+
+def share_storage(steps, nbytes, own=()) -> Dict[str, int]:
+    """field -> storage id for the fields written by ``steps``, a sequence of (reads, writes) in execution
+    order.  The fields in ``own`` come first, each with storage of its own.  Every other field takes the
+    storage of a field of the same byte size that no step at or after its own writer reads, else new
+    storage."""
+    last_read = {}
+    for idx, (reads, writes) in enumerate(steps):
+        for f in reads:
+            last_read[f] = idx
+    assign, next_id = {}, 0
+    free_pool = []            # (nbytes, storage id)
+    busy = []                 # (last read index, nbytes, storage id)
+    for name in own:
+        assign[name] = next_id
+        next_id += 1
+    for idx, (reads, writes) in enumerate(steps):
+        still = []
+        for (lr, nb, sid) in busy:
+            if lr < idx:
+                free_pool.append((nb, sid))
+            else:
+                still.append((lr, nb, sid))
+        busy = still
+        for f in writes:
+            if f in assign:
+                continue
+            nb = nbytes[f]
+            sid = None
+            for k, (pnb, psid) in enumerate(free_pool):
+                if pnb == nb:
+                    sid = psid
+                    free_pool.pop(k)
+                    break
+            if sid is None:
+                sid = next_id
+                next_id += 1
+            assign[f] = sid
+            busy.append((last_read.get(f, idx), nb, sid))
+    return assign
 
 
 class Plan:
@@ -154,44 +200,9 @@ class Plan:
         """field -> storage id.  Inputs and outputs own their storage; intermediates that cross
         pass boundaries share storage once dead (equal byte size only)."""
         fields = self.program.fields
-        launches = self.lowered.launches
-        first_write, last_read = {}, {}
-        for idx, l in enumerate(launches):
-            for f in l.writes:
-                first_write.setdefault(f, idx)
-            for f in l.reads:
-                last_read[f] = idx
-        assign, next_id = {}, 0
-        free_pool = []            # (nbytes, storage id)
-        busy = []                 # (last read index, nbytes, storage id)
-        for name in self.materialized_fields():
-            if fields[name].kind != "intermediate":
-                assign[name] = next_id
-                next_id += 1
-        for idx, l in enumerate(launches):
-            still = []
-            for (lr, nb, sid) in busy:
-                if lr < idx:
-                    free_pool.append((nb, sid))
-                else:
-                    still.append((lr, nb, sid))
-            busy = still
-            for f in l.writes:
-                if f in assign:
-                    continue
-                nb = fields[f].nbytes
-                sid = None
-                for k, (pnb, psid) in enumerate(free_pool):
-                    if pnb == nb:
-                        sid = psid
-                        free_pool.pop(k)
-                        break
-                if sid is None:
-                    sid = next_id
-                    next_id += 1
-                assign[f] = sid
-                busy.append((last_read.get(f, idx), nb, sid))
-        return assign
+        own = [name for name in self.materialized_fields() if fields[name].kind != "intermediate"]
+        return share_storage([(l.reads, l.writes) for l in self.lowered.launches],
+                             {name: f.nbytes for name, f in fields.items()}, own)
 
     def algorithmic_bytes(self) -> int:
         return self.lowered.algorithmic_bytes()
@@ -229,11 +240,19 @@ def plan_program(program: StencilProgram, options: Optional[PlanOptions] = None,
     if options.is_default:
         entry = lookup_tuned(program)
         if entry:
-            options = PlanOptions(**dict(entry["options"], peer_push=options.peer_push))
+            options = PlanOptions(**dict(entry["options"], peer_push=options.peer_push, cluster=options.cluster))
             tuned_from = entry.get("measured")
     lowered = lower_cuda.LoweredProgram(program)
     passes = []
     groups = None
+    if options.cluster and options.fuse and not options.peer_push:
+        from . import lower_cluster
+        layout = lower_cluster.ClusterLayout(program)
+        if layout.fits:
+            lower_cluster.lower_program_cluster(lowered, layout, specialize)
+            plan = Plan(program, lowered, [{"family": "cluster", "ops": [op.name for op in program.ops]}], options)
+            plan.tuned_from = tuned_from
+            return plan
     if options.fuse:
         try:
             from . import lower_stream
