@@ -330,6 +330,39 @@ def l2_hint_defines():
     return text
 
 
+# helpers of the passes over unaligned rows (Geometry.unaligned), emitted once after STREAM_PRELUDE
+UNALIGNED_PRELUDE = r"""
+// ---- unaligned rows: input cells copied by cp.async into the TMA ring, results stored cell by cell ----
+// one cell of a streamed input: flat element g of the field, zero when g lies outside the array (src-size 0)
+template <typename T>
+__device__ __forceinline__ void sf_cp_async(T* dst, const T* src, i64 g, i64 total) {
+    const bool in = (unsigned long long)g < (unsigned long long)total;
+    asm volatile("cp.async.ca.shared.global [%0], [%1], %2, %3;"
+                 ::"r"(sf_smem_addr(dst)), "l"(src + (in ? g : 0)), "n"((int)sizeof(T)), "r"(in ? (int)sizeof(T) : 0)
+                 : "memory");
+}
+// the slot's mbarrier counts one arrival per copying thread, made once all of that thread's copies have landed
+__device__ __forceinline__ void sf_cp_async_arrive(void* bar) {
+    asm volatile("cp.async.mbarrier.arrive.noinc.shared::cta.b64 [%0];" ::"r"(sf_smem_addr(bar)) : "memory");
+}
+#ifdef SF_STORE_HINT
+#define SF_STG_F32 "st.global.L2::cache_hint.f32 [%1], %2, %3;"
+#define SF_STG_F64 "st.global.L2::cache_hint.f64 [%1], %2, %3;"
+#else
+#define SF_STG_F32 "st.global.f32 [%1], %2;"
+#define SF_STG_F64 "st.global.f64 [%1], %2;"
+#endif
+// a row starts wherever (i * NJ + j) * NK puts it, so a cell is the widest store that is always aligned
+__device__ __forceinline__ void sf_stg1_if(bool on, float* p, float v) {
+    asm volatile("{\n\t.reg .pred q;\n\tsetp.ne.u32 q, %0, 0;\n\t@q " SF_STG_F32 "\n\t}"
+                 ::"r"((u32)on), "l"(p), "f"(v) SF_STG_HINT_ARG : "memory");
+}
+__device__ __forceinline__ void sf_stg1_if(bool on, double* p, double v) {
+    asm volatile("{\n\t.reg .pred q;\n\tsetp.ne.u32 q, %0, 0;\n\t@q " SF_STG_F64 "\n\t}"
+                 ::"r"((u32)on), "l"(p), "d"(v) SF_STG_HINT_ARG : "memory");
+}
+"""
+
 L2_HINT_DEFAULT = "3"
 ST64_DEFAULT = "0"
 SPLITBAR_DEFAULT = "0"
@@ -617,11 +650,16 @@ class GroupAnalysis:
 
 
 class Geometry:
-    def __init__(self, ana: GroupAnalysis, V, R, WR, WC, prefetch, KS=32, sync="cta", direct=False, tmem=False):
+    def __init__(self, ana: GroupAnalysis, V, R, WR, WC, prefetch, KS=32, sync="cta", direct=False, tmem=False,
+                 unaligned=False):
         """``KS`` = threads per tile row.  32 (a warp per row, k-neighbours by shuffle) in general;
         for groups without k-taps on a narrow innermost dimension the whole extent is one row of
-        ``KS = NK / V`` threads and thread t owns row group t / KS ("flat lanes": no idle lanes)."""
+        ``KS = NK / V`` threads and thread t owns row group t / KS ("flat lanes": no idle lanes).
+        ``unaligned``: the innermost rows are not a multiple of 16 bytes long, which a tiled TMA map of 2 or 3
+        dimensions needs for its strides.  The threads then copy the cells of the input planes themselves
+        (``cp.async``, see StreamKernelGen._emit_copy_issue) into the same shared-memory layout."""
         self.V, self.R, self.WR, self.WC, self.KS = V, R, WR, WC, KS
+        self.unaligned = bool(unaligned)
         self.NT = KS * WR * WC
         ktaps = any(i.col_reach for i in ana.fields.values())
         if KS != 32 and (WC != 1 or self.NT % 32 or (ktaps and KS not in (8, 16))):
@@ -643,7 +681,9 @@ class Geometry:
         # slots).  Only for inputs whose out-of-domain cells need no fix-up (TMA's zero fill is the
         # boundary value), 3-D tiles, CTA-wide synchronisation.
         self.direct = {}
-        if direct and ana.ndim == 3 and sync != "pair":
+        # (not with unaligned rows: the copies fill the cells outside a row with the neighbouring rows' data, and
+        # only the registers get the boundary value)
+        if direct and ana.ndim == 3 and sync != "pair" and not self.unaligned:
             for i in ana.ext_fields:
                 if i.row_ring and not i.col_ring and (i.bc is None or float(i.bc) == 0.0):
                     self.direct[i.name] = i.row_ring - 1
@@ -955,7 +995,10 @@ class StreamKernelGen:
         ext = a.ext_fields
         U = self.U
         stored = [i for i in a.fields.values() if i.stored]
-        params = ["const __grid_constant__ CUtensorMap tm_{}".format(n) for n in range(len(ext))]
+        if g.unaligned:
+            params = ["const {}* __restrict__ in_{}".format(T, n) for n in range(len(ext))]
+        else:
+            params = ["const __grid_constant__ CUtensorMap tm_{}".format(n) for n in range(len(ext))]
         params += ["{}* __restrict__ o_{}".format(T, n) for n in range(len(stored))]
         self.aux_name = {name: "x_{}".format(n) for n, name in enumerate(a.aux)}
         params += ["const {}* __restrict__ {}".format(T, self.aux_name[name]) for name in a.aux]
@@ -1004,8 +1047,8 @@ class StreamKernelGen:
                     T=T, f=self.fid[i.name], o=g.xcol_off[i.name]))
         e("unsigned long long* const bars = reinterpret_cast<unsigned long long*>(sf_smem + {});".format(g.bar_off))
         e("if (threadIdx.x == 0) {")
-        e("for (int s = 0; s < {}; ++s) sf_mbar_init(&bars[s], 1);".format(
-            g.D * (g.NW if g.pair else (2 if g.halves else 1))), 2)
+        e("for (int s = 0; s < {}; ++s) sf_mbar_init(&bars[s], {});".format(
+            g.D * (g.NW if g.pair else (2 if g.halves else 1)), self._copy_threads()[0] if g.unaligned else 1), 2)
         if self.split_barrier:
             e("sf_mbar_init(sf_smem + {}, {});".format(g.sbar_off, g.NT // 32), 2)
         for n in range(len(self.fbar) if self.flags else 0):
@@ -1083,6 +1126,8 @@ class StreamKernelGen:
         # in-domain mask of the owned cells, store mask of the owned rows
         e("u32 cmask = 0;")
         e("u32 smask = 0;")
+        if g.unaligned:
+            e("u32 stmask = 0;")
         e("#pragma unroll")
         e("for (int r = 0; r < {}; ++r) {{".format(R))
         if ndim == 3:
@@ -1094,6 +1139,9 @@ class StreamKernelGen:
         e("for (int v = 0; v < {}; ++v)".format(V), 2)
         e("if (rin && (gk + v) >= 0 && (gk + v) < {}) cmask |= 1u << (r * {} + v);".format(self.NK, V), 3)
         e("if (rst && c0 >= {} && c0 < {} && gk < {}) smask |= 1u << r;".format(g.HK0, g.TC - g.HK1, self.NK), 2)
+        if g.unaligned:
+            # store mask of the owned cells: the last vector of a row is ragged
+            e("if ((smask >> r) & 1u) stmask |= cmask & ({}u << (r * {}));".format((1 << V) - 1, V), 2)
         e("}")
         full_mask = (1 << (R * V)) - 1
         e("const bool interior = __syncthreads_and(cmask == {}u);".format(full_mask))
@@ -1102,6 +1150,8 @@ class StreamKernelGen:
         else:
             e("i64 out_off = (i64)gk - (i64)s_base * {NK};".format(NK=self.NK))
         e("asm volatile(\"\" : \"+r\"(cmask), \"+r\"(smask));   // keep them in registers: no re-derivation from blockIdx in the loop")
+        if g.unaligned:
+            e("asm volatile(\"\" : \"+r\"(stmask));")
         for n in range(len(stored)):
             e("{T}* ob_{n} = o_{n} + out_off;".format(T=T, n=n))
             e("asm volatile(\"\" : \"+l\"(ob_{n}));".format(n=n))
@@ -1125,7 +1175,18 @@ class StreamKernelGen:
         # one elected lane of warp 0 arms the mbarrier; with many boxes per plane (wide 2-D tiles) the
         # copies themselves are issued by the first `issuers` warps, one box each per round
         issuers = 1 if total_boxes <= 2 else min(nwarps, nbox)
-        if g.pair:
+        if g.unaligned:
+            # every thread of a barrier's group copies its share of the group's part of the plane
+            if g.halves:
+                e("const u32 upper_u = warp_u >= {} ? 1u : 0u;              // which half of the tile this warp belongs to".format(nwarps // 2))
+                e("const u32 seam_lo = warp_u == {} ? 1u : 0u, seam_hi = warp_u == {} ? 1u : 0u;".format(nwarps // 2 - 1, nwarps // 2))
+                e("unsigned long long* const wbars = bars + upper_u * {};".format(g.D))
+            elif g.pair:
+                e("unsigned long long* const wbars = bars + warp_u * {};".format(g.D))
+            else:
+                e("unsigned long long* const wbars = bars;")
+            self._emit_copy_issue(ext)
+        elif g.pair:
             # every warp stages its own rows (3-D) / columns (2-D) of the plane and owns the barriers
             box_elems = g.box[0] * g.box[1]
             e("unsigned long long* const wbars = bars + warp_u * {};".format(g.D))
@@ -1182,11 +1243,13 @@ class StreamKernelGen:
                 if issuers > 1:
                     e("}", 2)
             e("};")
-        if g.halves:
+        if g.unaligned:
+            e("const bool issuer = true;                  // (every thread copies its share of a plane)")
+        elif g.halves:
             e("const bool issuer = (warp_u % {}) == 0;            // the first warp of each half".format(nwarps // 2))
         else:
             e("const bool issuer = warp_u < {};".format(issuers))
-        e("if (issuer && sf_elect_one()) {")
+        e("if (issuer) {" if g.unaligned else "if (issuer && sf_elect_one()) {")
         if static_d:
             e("for (int p = 0; p < {}; ++p) if (t_begin + p < t_end) issue(t_begin + p, p);".format(g.P), 2)
         else:
@@ -1297,7 +1360,10 @@ class StreamKernelGen:
         name = "sf_stream_{}".format(digest)
         src = ("extern \"C\" __global__ void __launch_bounds__({}, 1)\n{}({})\n{{\n{}\n}}\n".format(
             g.NT, name, ", ".join(params), body))
-        args = [("tmap", {"field": i.name, "box": self._box()}) for i in ext]
+        if g.unaligned:
+            args = [("buf", i.name) for i in ext]
+        else:
+            args = [("tmap", {"field": i.name, "box": self._box()}) for i in ext]
         args += [("buf", i.name) for i in stored]
         args += [("buf", name) for name in a.aux]
         args += [("scalar", self.program.fields[s].data_type, s) for s in self.scalars]
@@ -1391,10 +1457,60 @@ class StreamKernelGen:
 
     def _needs_fixup(self, info):
         """Cells outside the domain must read as the boundary value.  Input planes arrive through TMA,
-        which zero-fills everything outside the tensor, so a zero boundary value needs no code."""
+        which zero-fills everything outside the tensor, so a zero boundary value needs no code -- except with
+        unaligned rows: the cell copies only zero-fill past the ends of the whole array, and the cells left and
+        right of a row and in the rows beyond the domain's edges hold neighbouring rows' data."""
         if not info.consumed or info.bc is None:
             return False
-        return not (info.kind == "ext" and float(info.bc) == 0.0)
+        return not (info.kind == "ext" and float(info.bc) == 0.0 and not self.geo.unaligned)
+
+    def _copy_threads(self):
+        """Unaligned rows: (threads that copy for one mbarrier, C expression of a thread's rank among them)."""
+        g = self.geo
+        if g.pair:
+            return 32, "(int)(threadIdx.x & 31)"
+        if g.halves:
+            return g.NT // 2, "(int)(threadIdx.x % {})".format(g.NT // 2)
+        return g.NT, "(int)threadIdx.x"
+
+    def _emit_copy_issue(self, ext):
+        """Unaligned rows: ``issue(t, s)`` copies the cells of every streamed input's plane that the calling thread's
+        mbarrier group stages (the whole tile; a warp's rows or columns with ``pair``; a half's rows with
+        ``halves``) into ring slot s, one ``cp.async`` per cell, the threads of the group taking turns.  Cells
+        outside the array are zero-filled; a thread arrives on the slot's mbarrier once its copies have landed.
+        Row starts are anywhere in memory, so no copy wider than a cell is aligned in general.  (One rank-1 TMA
+        box per tile row, started at such an address, stopped the first kernel that used it with an illegal
+        instruction on a B200: DESIGN 3.2.)"""
+        g, a, e = self.geo, self.ana, self.emit
+        nthr, tid = self._copy_threads()
+        if g.pair and a.ndim == 3:
+            row0, nrows, col0, ncols = "warp_u * {}".format(g.warp_rows), g.warp_rows, "0", g.TC
+        elif g.pair:
+            row0, nrows, col0, ncols = "0", 1, "warp_u * {}".format(g.box[0]), g.box[0]
+        elif g.halves:
+            row0, nrows, col0, ncols = "(int)upper_u * {}".format(g.TR // 2), g.TR // 2, "0", g.TC
+        else:
+            row0, nrows, col0, ncols = "0", (g.TR if a.ndim == 3 else 1), "0", g.TC
+        plane = self.NJ * self.NK if a.ndim == 3 else self.NK
+        e("auto issue = [&](int t, int s) {")
+        for n, i in enumerate(ext):
+            e("{", 2)
+            if a.ndim == 3:
+                e("const i64 pb = (i64)(t - ({lag}) - s_base) * {pl} + (i64)(tile_j0 - {HJ0} + {row0}) * {NK} + tile_k0 - {HK0} + {col0};".format(
+                    lag=i.lag, pl=plane, HJ0=g.HJ0, row0=row0, NK=self.NK, HK0=g.HK0, col0=col0), 3)
+            else:
+                e("const i64 pb = (i64)(t - ({lag}) - s_base) * {pl} + tile_k0 - {HK0} + {col0};".format(
+                    lag=i.lag, pl=plane, HK0=g.HK0, col0=col0), 3)
+            e("#pragma unroll 1", 3)
+            e("for (int q = {tid}; q < {n}; q += {nthr}) {{".format(tid=tid, n=nrows * ncols, nthr=nthr), 3)
+            e("const int r = q / {c}, c = q - r * {c};".format(c=ncols), 4)
+            e("sf_cp_async(tile_{f} + s * {sz} + ({row0} + r) * {TC} + {col0} + c, in_{n}, pb + (i64)r * {NK} + c, {tot}ll);".format(
+                f=self.fid[i.name], sz=g.TR * g.TC, row0=row0, TC=g.TC, col0=col0, n=n, NK=self.NK,
+                tot=self.NS * plane), 4)
+            e("}", 3)
+            e("}", 2)
+        e("sf_cp_async_arrive(&wbars[s]);", 2)
+        e("};")
 
     def _emit_steps(self, ext, static_d):
         g, a, e, U = self.geo, self.ana, self.emit, self.U
@@ -1419,7 +1535,10 @@ class StreamKernelGen:
                 # published them: the arrivals of the previous step on the streamed inputs' barriers
                 for i in ext:
                     self._flag_wait(i, 1, u)
-            e("if (issuer && t + {P} < t_end) {{ if (sf_elect_one()) issue(t + {P}, {nxt}); }}".format(P=g.P, nxt=nxt), 2)
+            if g.unaligned:
+                e("if (issuer && t + {P} < t_end) issue(t + {P}, {nxt});".format(P=g.P, nxt=nxt), 2)
+            else:
+                e("if (issuer && t + {P} < t_end) {{ if (sf_elect_one()) issue(t + {P}, {nxt}); }}".format(P=g.P, nxt=nxt), 2)
             last_comm = self._emit_ops(u, ext, ph, self.ops_limit)
             if g.pair:
                 e("sf_sync_neighbours<{}>(warp_u);".format(g.NW), 2)
@@ -1862,9 +1981,15 @@ class StreamKernelGen:
                 T=T, n=idx, p=plane, stride=(self.NJ * self.NK if a.ndim == 3 else self.NK)), 3)
             e("asm volatile(\"\" : \"+l\"(op));              // one address computation for all rows", 3)
             e("const bool inchunk = ({p}) >= c_begin && ({p}) < c_end;".format(p=plane), 3)
-            for r in range(R):
-                e("sf_stg_if(inchunk && ({sm} & {m}u), op + {o}, nv[{r}]);".format(
-                    sm="smask", m=1 << r, o=r * self.NK, r=r), 3)
+            if g.unaligned:
+                for r in range(R):
+                    for v in range(V):
+                        e("sf_stg1_if(inchunk && ((stmask >> {b}) & 1u), op + {o}, {c});".format(
+                            b=r * V + v, o=r * self.NK + v, c=self.cellref("nv[{}]".format(r), v)), 3)
+            else:
+                for r in range(R):
+                    e("sf_stg_if(inchunk && ({sm} & {m}u), op + {o}, nv[{r}]);".format(
+                        sm="smask", m=1 << r, o=r * self.NK, r=r), 3)
         self._finish_field(info, plane, u)
         e("}", 2)
 
@@ -2126,7 +2251,16 @@ def _vector_width(program, dtype, options=None):
     want = getattr(options, "vector", 0) or v
     if want > v and want % v == 0 and program.shape[-1] % (want * 32) == 0:
         v = want
-    return v if program.shape[-1] % v == 0 else None
+    if program.shape[-1] % v == 0 or unaligned_rows(program, dtype, options):
+        return v                    # (unaligned rows: the last vector of a row is ragged)
+    return None
+
+
+def unaligned_rows(program, dtype, options):
+    """True when a group of ``dtype`` fields is streamed in unaligned-row mode (``PlanOptions.unaligned``): its
+    innermost rows are not a multiple of 16 bytes long, and the plan allows it (not in slab mode)."""
+    return bool(getattr(options, "unaligned", 0) and not getattr(options, "peer_push", False)
+                and (program.shape[-1] * dtype.bytes) % 16 != 0)
 
 
 def candidate_geometries(program, ops, options):
@@ -2265,6 +2399,8 @@ def choose_geometry(program, ops, options):
         wide.vector = 32 // ops[0].data_type.bytes
         trials = [wide, options]
     best = None
+    # (the cost model prices a pass over unaligned rows like an aligned one)
+    unaligned = unaligned_rows(program, ops[0].data_type, options)
     for opts in trials:
         try:
             V, candidates = candidate_geometries(program, ops, opts)
@@ -2284,16 +2420,18 @@ def choose_geometry(program, ops, options):
                         sync = getattr(opts, "sync", "") or DEFAULT_SYNC
                         direct = bool(getattr(opts, "direct", 0))
                         tmem = int(getattr(opts, "tmem", 0) or 0)
-                        geo = Geometry(ana, V, R, WR, WC, prefetch, KS, sync, direct=direct, tmem=bool(tmem))
+                        geo = Geometry(ana, V, R, WR, WC, prefetch, KS, sync, direct=direct, tmem=bool(tmem),
+                                       unaligned=unaligned)
                         if geo.tmem and tmem < 2 and ana.register_estimate(R, V) < register_limit(geo.NT):
                             # the windows fit the registers: nothing to park (tmem = 2 parks all the same, so
                             # that the tensor-memory code of passes far from their register limit can be tested)
-                            geo = Geometry(ana, V, R, WR, WC, prefetch, KS, sync, direct=direct)
+                            geo = Geometry(ana, V, R, WR, WC, prefetch, KS, sync, direct=direct, unaligned=unaligned)
                         elif geo.tmem and not getattr(opts, "sync", ""):
                             # a pass at its register limit spends what the parked planes free on per-field
                             # mbarriers instead of the CTA barrier (Jacobi-3D 1024^3: 3.69 vs 3.84 ms; parked
                             # planes under the CTA barrier alone: 4.04 ms, profiles/r03_sweep_tmem_config1.txt)
-                            geo = Geometry(ana, V, R, WR, WC, prefetch, KS, "flags", direct=direct, tmem=True)
+                            geo = Geometry(ana, V, R, WR, WC, prefetch, KS, "flags", direct=direct, tmem=True,
+                                           unaligned=unaligned)
                     except NotStreamable:
                         break
                     if geo.smem > SMEM_LIMIT:
@@ -2541,10 +2679,14 @@ def lower_group(lowered: LoweredProgram, ops: List[StencilOp], options, speciali
     if chosen is None:
         raise NotStreamable("group cannot stream")
     ana, geo = chosen
+    # the cell copies of unaligned rows index the whole field (all NS planes, zero-fill past its ends): a slab buffer,
+    # which holds only some planes, would be read past its end -- unaligned_rows() keeps the mode out of slab mode
+    assert not (geo.unaligned and getattr(options, "peer_push", False))
     gen = StreamKernelGen(program, ops, ana, geo, specialize, peer_push=bool(getattr(options, "peer_push", 0)))
     name, src, args = gen.generate()
     if name not in lowered.kernels:
-        lowered.kernels[name] = KernelSpec(name, src, (geo.NT, 1, 1), "streamed")
+        lowered.kernels[name] = KernelSpec(name, src, (geo.NT, 1, 1), "streamed",
+                                           prelude=UNALIGNED_PRELUDE if geo.unaligned else "")
     NI, NJ, NK = program.shape3
     n_stream = program.shape[0]
     gx = -(-NK // geo.BK)
@@ -2617,6 +2759,8 @@ def lower_group(lowered: LoweredProgram, ops: List[StencilOp], options, speciali
                               "tile_efficiency": _tile_efficiency(ana, geo),
                               "fwd": ana.max_lag,
                               "chunk_fn": chunk_for, "work_fn": work_table, "work_items_fn": work_items})
+    if geo.unaligned:
+        launch.info["unaligned"] = True       # (recorded for the passes that run so only: other records stay as they were)
     lowered.launches.append(launch)
     lowered.uses_stream = True
     return launch

@@ -102,7 +102,7 @@ class PlanOptions:
 
     def __init__(self, fuse=None, max_depth=None, rows_per_thread=None, warps=None, chunk=None,
                  prefetch=None, vector=None, threads_per_row=None, sync=None, direct=None, tmem=None,
-                 peer_push=None, cluster=None):
+                 peer_push=None, cluster=None, unaligned=None):
         env = os.environ
         self.is_default = (all(v is None for v in (fuse, max_depth, rows_per_thread, warps, chunk, prefetch, vector,
                                                    threads_per_row, sync, direct, tmem))
@@ -128,6 +128,11 @@ class PlanOptions:
         # part in ``is_default`` and survives the replacement of the options by a measured plan.  Ignored with
         # fuse=False and in slab mode.
         self.cluster = int(env.get("SFB200_CLUSTER", "0")) if cluster is None else int(cluster)
+        # 1: groups whose innermost row is not a multiple of 16 bytes stream too: the threads copy their input cells
+        # into the shared-memory ring with cp.async (a tiled TMA map needs 16-byte row strides), and results leave by
+        # single-cell stores (lower_stream).  0: such groups run as one-operator kernels.  Programs with aligned rows
+        # get the same kernels either way.  Like ``cluster`` not a tuning knob; ignored with fuse=False and in slab mode.
+        self.unaligned = int(env.get("SFB200_UNALIGNED", "0")) if unaligned is None else int(unaligned)
         # slab mode (set by distributed.SlabProgram): streamed kernels store the edge planes of their
         # results straight into the neighbouring GPUs' halo planes.  Not a tuning knob: it does not
         # take part in ``is_default`` and survives the replacement of the options by a measured plan.
@@ -240,7 +245,8 @@ def plan_program(program: StencilProgram, options: Optional[PlanOptions] = None,
     if options.is_default:
         entry = lookup_tuned(program)
         if entry:
-            options = PlanOptions(**dict(entry["options"], peer_push=options.peer_push, cluster=options.cluster))
+            options = PlanOptions(**dict(entry["options"], peer_push=options.peer_push, cluster=options.cluster,
+                                         unaligned=options.unaligned))
             tuned_from = entry.get("measured")
     lowered = lower_cuda.LoweredProgram(program)
     passes = []
