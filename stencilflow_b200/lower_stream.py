@@ -32,7 +32,7 @@ from typing import Dict, List, Optional, Tuple
 
 from . import dtypes
 from . import expr as ex
-from .lower_cuda import (KernelSpec, LaunchSpec, LoweredProgram, _MATH_F32, _MATH_F64, ctype_of,
+from .lower_cuda import (KernelSpec, LaunchSpec, LoweredProgram, _MATH_F32, _MATH_F64, ctype_of, value_literal,
                          literal)
 from .stencil_op import JUNK_VAL, StencilOp, StencilProgram
 
@@ -437,6 +437,7 @@ class GroupAnalysis:
         self.aux_reach: Dict[str, List[int]] = {}            # name -> [back, fwd] along the streamed dim
         self.aux_bc: Dict[str, float] = {}
         self.copy_taps = set()                               # (operator, field) read with a ``copy`` boundary
+        self.copy_reach = {}                                 # copy_taps -> (min, max) offset along the streamed dim
         produced = {op.name for op in ops}
         # fields of the group that operators outside it read: they have to be written to HBM
         later = set()
@@ -485,6 +486,8 @@ class GroupAnalysis:
                             raise NotStreamable("consumers of {} disagree on the boundary handling".format(field))
                         info.copy = True
                         self.copy_taps.add((op.name, field))
+                        ds = [t[1] for t in taps if t[0] == field]
+                        self.copy_reach[(op.name, field)] = (min(ds + [0]), max(ds + [0]))
                         if (field, 0, 0, 0) not in taps:
                             taps.append((field, 0, 0, 0))
                     else:
@@ -1260,6 +1263,10 @@ class StreamKernelGen:
         # ``copy`` boundaries are resolved by the consuming operator: its trips near the border need the code too
         needs_bc += [a.fields[op] for (op, _) in sorted(a.copy_taps) if a.fields[op] not in needs_bc]
         needs_bc += [a.fields[f] for (_, f) in sorted(a.copy_taps) if a.fields[f] not in needs_bc]
+        # a trip without boundary code needs the planes of an operator's copy taps inside the domain as well: the
+        # operator at plane t - lag reads plane t - lag + d
+        back = [i.lag for i in needs_bc] + [a.fields[op].lag - lo for (op, _), (lo, _) in a.copy_reach.items()]
+        ahead = [i.lag for i in needs_bc] + [a.fields[op].lag - hi for (op, _), (_, hi) in a.copy_reach.items()]
         def emit_loop(n_ops):
             self.ops_limit = n_ops
             flip = static_d and (U // g.D) % 2 == 1
@@ -1269,8 +1276,8 @@ class StreamKernelGen:
                 # loops -- runs of fast trips, single trips with the boundary code in between -- rather than the
                 # two arms of a branch inside one loop: the register assignment of the fast loop is then its own
                 # (no copies at the join of the arms: 57 MOV per trip of the Jacobi-3D pass)
-                lag_max = max(i.lag for i in needs_bc)
-                lag_min = min(i.lag for i in needs_bc)
+                lag_max = max(back)
+                lag_min = min(ahead)
                 cond = "__all_sync(0xffffffffu, interior && (t0 - ({}) >= 0) && (t0 + {} - ({}) < {}))".format(
                     lag_max, U - 1, lag_min, self.NS)
                 e("int t0 = t_begin;")
@@ -1297,8 +1304,8 @@ class StreamKernelGen:
                 e("for (int t0 = t_begin; t0 < t_end; t0 += {}) {{".format(U))
                 variants = [True]
                 if needs_bc and self.fast_path:
-                    lag_max = max(i.lag for i in needs_bc)
-                    lag_min = min(i.lag for i in needs_bc)
+                    lag_max = max(back)
+                    lag_min = min(ahead)
                     e("const bool fast = __all_sync(0xffffffffu, interior && (t0 - ({}) >= 0) && (t0 + {} - ({}) < {}));".format(
                         lag_max, U - 1, lag_min, self.NS), 2)
                     variants = [False, True]
@@ -2001,6 +2008,7 @@ class StreamKernelGen:
         for r in range(g.R):
             for v in range(g.V):
                 local = {}
+                assigned = collections.Counter()
                 for s in op.statements:
                     rhs = ex.emit_c(
                         s.value,
@@ -2013,8 +2021,11 @@ class StreamKernelGen:
                         local_ids[s.target] = len(local_ids)
                     lname = "q{}_{}_{}".format(local_ids[s.target], r, v)
                     ty = "const bool" if isinstance(s.value, (ex.Cmp, ex.Logic)) else "const " + T
-                    if s.target in local:
-                        lname += "b"
+                    # a fresh name per assignment: q..., q...b, q...b2, ...
+                    n = assigned[s.target]
+                    if n:
+                        lname += "b" if n == 1 else "b{}".format(n)
+                    assigned[s.target] += 1
                     e("{} {} = {};".format(ty, lname, rhs), 3)
                     local[s.target] = lname
                 target = op.name if op.name in local else op.statements[-1].target
@@ -2226,9 +2237,9 @@ class StreamKernelGen:
         if name in local:
             return local[name]
         if name in self.specialize:
-            return self.lit(self.specialize[name])
+            return value_literal(self.specialize[name], self.ct)
         if name in self.program.constants:
-            return self.lit(self.program.constants[name]["value"])
+            return value_literal(self.program.constants[name]["value"], self.ct)
         if name in self.sc_name:
             return "({}){}".format(self.T, self.sc_name[name])
         raise NameError("Unknown name {} in operator {}".format(name, op.name))
